@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- drone-steps/s of the fused Physics.DYN control tick on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, weak scaling)
 
 Workload (config.workload): BASELINE configs[2] -- MultiHoverAviary, 65536 drones per GPU as 32768 two-drone
@@ -10,13 +10,19 @@ step), random actions in [-1,1], SAME_STEP autoreset (an RL rollout).  One "step
 the fused kernel over all 65536 drones of the rank.  The working set of one batch (42 MB) fits the 126 MB L2, so the
 timed loop rotates over R independent batches (R x 42 MB > L2): every launch finds its inputs in HBM.
 
-JSON keys follow the driver contract; `value` = device-resident steps (actions already in HBM; the K-step window is
-repeated until >= 50 ms have been timed and the median window is reported, per-rank values alongside), `e2e` = the same
+One JSON line; `value` = device-resident steps (actions already in HBM; after W warm-up steps exactly K steps are timed
+in one window, the slowest rank's window counts, per-rank values alongside), `e2e` = the same
 steps through the NumPy API (pinned H2D of the actions + D2H of obs/reward/flags/terminal observations inside the timed
 region) with the pinned D2H copy rate measured in the same run (`pcie_frac`), `roofline` = algorithmic bytes of the step
-kernel / its launch period in the timed loop (`frac`, back-to-back launches overlap through programmatic dependent
+kernel / its launch period in the timed window (`frac`, back-to-back launches overlap through programmatic dependent
 launch) and / its duration alone on an idle GPU with a cold L2 (`frac_isolated`), against MEASURED_PEAKS.json;
 `cpu_baseline` = the float64 NumPy oracle on a bounded sample on this host.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy: obs [E, D, 72], reward [E],
+terminated / truncated / final_obs_mask [E] (as float32), and final_obs [E, D, 72], the terminal observation of every
+aviary that finished in that step and zeros for the others, so every array has the same shape in every run.  Actions come
+from a seeded generator and the step count is fixed by W and K, so two builds run with the same arguments can be compared
+array for array.
 """
 import argparse
 import json
@@ -50,8 +56,11 @@ def parse():
     ap.add_argument("--batches", type=int, default=8, help="independent 65536-drone batches rotated through (L2 defeat)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
-    ap.add_argument("--min-ms", type=float, default=50.0, help="repeat the K-step window until this much device time has been timed")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def bind_to_gpu_numa(local):
@@ -187,6 +196,25 @@ def reference_arm(a):
     }))
 
 
+def step_outputs(result):
+    """Device copies of what one vector-API step returned, taken before later steps reuse its buffers."""
+    import torch
+    obs, rew, term, trunc, info = result
+    out = {"obs": obs.clone(), "reward": rew.clone(), "terminated": term.clone(), "truncated": trunc.clone()}
+    if "final_obs" in info:
+        mask = info["_final_obs"]
+        out["final_obs_mask"], out["final_obs"] = mask.clone(), torch.where(mask[:, None, None], info["final_obs"], 0.0)
+    return out
+
+
+def dump_outputs(directory, outputs):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        x = t.cpu().numpy()
+        np.save(os.path.join(directory, name + ".npy"), x if x.dtype in (np.float32, np.float64) else x.astype(np.float32))
+
+
 def workload_config(a, drones_per_step):
     return {"workload": "MultiHoverAviary x %d aviaries x %d drones (=%d drones per GPU), act=RPM (A=4), action buffer B=15, obs 72 f32, "
                         "pyb 240 Hz / ctrl 30 Hz (S=8), random actions, SAME_STEP autoreset [BASELINE configs[2]]" % (DRONES_PER_GPU // D, D, DRONES_PER_GPU),
@@ -261,42 +289,33 @@ def main():
         return [float(o.item()) for o in out]
 
     def run(n, k0=0):
+        res = None
         for k in range(k0, k0 + n):
             i = k % R
-            envs[i].step(acts[i][(k // R) % K_ACT])
+            res = envs[i].step(acts[i][(k // R) % K_ACT])
+        return res
 
-    # ---- device-resident throughput: windows of exactly K steps, barrier + sync on both sides, max over ranks per window ----
+    # ---- device-resident throughput: one window of exactly K steps, barrier + sync on both sides, max over ranks ----
     run(max(a.warmup, 3))
-    windows, total_ms, k0 = [], 0.0, a.warmup
+    k0 = a.warmup
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local) as clk:
-        while (total_ms < a.min_ms or not windows) and len(windows) < 2000:
-            barrier()
-            ev0.record()
-            run(a.steps, k0)
-            ev1.record()
-            barrier()
-            w = all_max(ev0.elapsed_time(ev1))
-            windows.append(w)
-            total_ms += w
-            k0 += a.steps
+        barrier()
+        ev0.record()
+        last = run(a.steps, k0)
+        ev1.record()
+        barrier()
+        my_ms = ev0.elapsed_time(ev1)
+        outputs = step_outputs(last) if a.dump_outputs and rank == 0 else None
+        k0 += a.steps
         # keep the sampler over a little more load so short runs still see clocks under load
         t_end = time.time() + 0.6
         while time.time() < t_end:
             run(50)
         torch.cuda.synchronize()
-    ms_window = statistics.median(windows)
+    ms_window = all_max(my_ms)
     value = DRONES_PER_GPU * world * a.steps / (ms_window * 1e-3)
-    my_ms = []      # this rank's own windows (not max-reduced) for the per-rank report
-    for _ in range(min(len(windows), 20)):
-        torch.cuda.synchronize()
-        ev0.record()
-        run(a.steps, k0)
-        ev1.record()
-        torch.cuda.synchronize()
-        my_ms.append(ev0.elapsed_time(ev1))
-        k0 += a.steps
-    per_rank = all_gather_f(DRONES_PER_GPU * a.steps / (statistics.median(my_ms) * 1e-3))
+    per_rank = all_gather_f(DRONES_PER_GPU * a.steps / (my_ms * 1e-3))
 
     # ---- roofline of the step kernel: launch period in the timed loop (pipelined) and duration alone (isolated, cold L2) ----
     peaks = {}
@@ -305,14 +324,7 @@ def main():
     except Exception:
         pass
     peak_gbs = float(peaks.get("hbm_gbs", 6650.0))
-    n_long = max(a.steps, 1000)
-    torch.cuda.synchronize()
-    ev0.record()
-    run(n_long, k0)
-    ev1.record()
-    torch.cuda.synchronize()
-    kern_ms = ev0.elapsed_time(ev1) / n_long                 # back-to-back launches of only this kernel: launch period
-    k0 += n_long
+    kern_ms = my_ms / a.steps                                 # back-to-back launches of only this kernel: launch period
     scrub = torch.empty(192 << 20, dtype=torch.uint8, device=dev)
     iso = []
     for k in range(40):
@@ -335,9 +347,9 @@ def main():
                 "frac": alg / (kern_ms * 1e-3) / 1e9 / peak_gbs, "frac_isolated": alg / (iso_ms * 1e-3) / 1e9 / peak_gbs,
                 "traffic": traffic, "kernel": "step_fast_kernel<A=4,task,reset,rpy_f32>", "kernel_ms": kern_ms, "kernel_ms_isolated": iso_ms,
                 "alg_bytes_per_drone_step": ALG_BYTES, "alg_bytes_per_launch": alg,
-                "timing": "frac: CUDA events around %d back-to-back launches / count (launch period; neighbours overlap through programmatic "
-                          "dependent launch); frac_isolated: median of events around single launches after a sync and a 192 MB L2 scrub "
-                          "(includes ~2 us of event/launch gap); traffic: ncu dram__bytes_read+write per launch (profiles/)" % n_long,
+                "timing": "frac: CUDA events around the %d back-to-back launches of the timed window / count (launch period; neighbours overlap "
+                          "through programmatic dependent launch); frac_isolated: median of events around single launches after a sync and a "
+                          "192 MB L2 scrub (includes ~2 us of event/launch gap); traffic: ncu dram__bytes_read+write per launch (profiles/)" % a.steps,
                 "peak_source": "MEASURED_PEAKS.json (of measured)" if peaks else "fallback 6.65 TB/s (of fallback)"}
 
     # ---- end to end through the NumPy API: page-locked ndarray actions in, ndarrays out, every copy inside step() ----
@@ -439,8 +451,7 @@ def main():
             "dtype": "f64", "data": "synthetic", "config": workload_config(a, DRONES_PER_GPU * world),
             "clocks": clk.summary(),
             "e2e": e2e,
-            "gpu_launches": a.steps * len(windows),
-            "timed_windows": {"count": len(windows), "steps_each": a.steps, "total_ms": total_ms, "ms_min": min(windows), "ms_median": ms_window, "ms_max": max(windows)},
+            "gpu_launches": a.steps,
             "per_rank_value": per_rank,
             "roofline": roofline,
             "substeps_per_s": value * S,
@@ -450,6 +461,8 @@ def main():
         if world == 1 and not a.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baseline_single()
         print(json.dumps(out))
+    if outputs is not None:
+        dump_outputs(a.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 

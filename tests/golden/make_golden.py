@@ -262,6 +262,7 @@ def main():
                                        gnd_thrust=gnd, drag_body=drag_body, downwash_body_z=dw)))
     save("effects_formula", **out)
     adjacency_fixture()
+    logger_fixture()
 
 
 def adjacency_fixture():
@@ -275,6 +276,27 @@ def adjacency_fixture():
             env = R.CtrlAviary(num_drones=nd, neighbourhood_radius=radius, initial_xyzs=xyz, physics=R.Physics.DYN)
         out.update(flat("case%d" % k, dict(pos=env.pos.copy(), radius=np.float64(radius), adjacency=env._getAdjacencyMatrix())))
     save("adjacency", **out)
+
+
+def logger_fixture():
+    """utils/Logger.py: the arrays the reference's Logger holds after 7 ticks of 3 drones, logged one drone at a time."""
+    import tempfile
+    import types
+    for name in ("matplotlib", "matplotlib.pyplot", "cycler"):          # plotting deps of the reference module; unused here
+        sys.modules.setdefault(name, types.ModuleType(name))
+    sys.modules["cycler"].cycler = lambda *a, **k: None
+    from gym_pybullet_drones.utils.Logger import Logger
+    T, nd = 7, 3
+    rng = np.random.default_rng(1)
+    timestamp, state, control = np.arange(T) / 48, np.zeros((T, nd, 20)), np.zeros((T, nd, 12))
+    with tempfile.TemporaryDirectory() as tmp:
+        lg = Logger(logging_freq_hz=48, output_folder=os.path.join(tmp, "r"), num_drones=nd)
+        for t in range(T):
+            for j in range(nd):
+                state[t, j], control[t, j] = rng.normal(size=20), rng.normal(size=12)
+                lg.log(drone=j, timestamp=timestamp[t], state=state[t, j], control=control[t, j])
+    save("logger_reference", timestamp=timestamp, state=state, control=control,
+         timestamps=lg.timestamps, states=lg.states, controls=lg.controls)
 
 
 if __name__ == "__main__":

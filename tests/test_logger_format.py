@@ -1,5 +1,5 @@
-"""Logger writes the reference's on-disk layout (SURVEY.md 8f rank 4); checked against the reference's own Logger when it
-is importable in this container (needs nothing GPU)."""
+"""Logger writes the reference's on-disk layout (SURVEY.md 8f rank 4); checked against arrays recorded from the reference's
+own Logger (tests/golden/logger_reference.npz, made by tests/golden/make_golden.py).  CPU only."""
 import os
 
 import numpy as np
@@ -28,23 +28,13 @@ def test_logger_layout_and_roundtrip(tmp_path):
         lg.log(drone=3, timestamp=0, state=states[0, 0])
 
 
-def test_logger_matches_reference_logger(tmp_path):
-    from oracle.ref_loader import reference_available
-    if not reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    import sys
-    import types
-    for name in ("matplotlib", "matplotlib.pyplot", "cycler"):          # plotting deps of the reference module; unused here
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules["cycler"].cycler = lambda *a, **k: None
-    from oracle.ref_loader import load_reference
-    load_reference()
-    from gym_pybullet_drones.utils.Logger import Logger as RefLogger
-    a, b = RefLogger(logging_freq_hz=48, output_folder=str(tmp_path / "r"), num_drones=3), Logger(logging_freq_hz=48, output_folder=str(tmp_path / "m"), num_drones=3)
-    rng = np.random.default_rng(1)
-    for t in range(7):
-        for j in range(3):
-            s, c = rng.normal(size=20), rng.normal(size=12)
-            a.log(drone=j, timestamp=t / 48, state=s, control=c)
-            b.log(drone=j, timestamp=t / 48, state=s, control=c)
-    assert np.array_equal(a.timestamps, b._trimmed()[0]) and np.array_equal(a.states, b._trimmed()[1]) and np.array_equal(a.controls, b._trimmed()[2])
+def test_logger_matches_reference_logger(golden, tmp_path):
+    """The reference's Logger fed the same entries, one drone at a time, holds the same arrays."""
+    g = golden("logger_reference")
+    nd = g["state"].shape[1]
+    lg = Logger(logging_freq_hz=48, output_folder=str(tmp_path), num_drones=nd)
+    for t in range(len(g["timestamp"])):
+        for j in range(nd):
+            lg.log(drone=j, timestamp=g["timestamp"][t], state=g["state"][t, j], control=g["control"][t, j])
+    ts, st, ct = lg._trimmed()
+    assert np.array_equal(ts, g["timestamps"]) and np.array_equal(st, g["states"]) and np.array_equal(ct, g["controls"])
